@@ -20,9 +20,13 @@ FASTQ packing, FASTQ landing in the library's pinned host ring.
               configs[1] cell (5.3 GB of FASTQ per step; the full cell would need 394 GB of scratch disk per step).
   configs1  : BASELINE configs[1] (250 Mb haploid, PE150 10x) on rank 0's GPU, the round-1 headline, kept for continuity.
 
---impl reference times the reference's own CPU implementation (oracle/_ref/bin/scssim, built from /root/reference by
-oracle/build_ref.sh) with all host threads; every step is one whole `scssim genreads` process on a bounded sample of the same
+--impl reference times the reference's own CPU implementation (oracle/_ref/bin/scssim, built by oracle/build_ref.sh from the
+SCSsim sources at BASELINE.json's reference_path or $SCS_REFERENCE_DIR) with all host threads; every step is one whole `scssim genreads` process on a bounded sample of the same
 workload (a 1/387-scale cell: same GC spectrum, gamma, coverage, profile, layout), and the line says "extrapolated".
+
+--dump-outputs DIR keeps a fixed sample of the FASTQ that the last timed step produced (FastqSample) and writes it as DIR/*.npy, so
+that two builds run with the same arguments can be compared output for output. That step hands its slabs to a Python sink instead of
+the null sink, inside the timed region, so the line of such a run says "dump_outputs": true in its detail and is not the headline.
 """
 import argparse
 import ctypes as C
@@ -34,7 +38,10 @@ import tempfile
 import threading
 import time
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True   # the tree may be read-only; nothing is written into it
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -71,6 +78,40 @@ def bench_config(scale, coverage):
     return {"workload": name, "layout": "PE", "read_length": READ_LEN, "coverage_flag": coverage, "gamma": GAMMA, "isize": ISIZE,
             "genome_bases": N_CHROM * 2 * clen, "reads_per_step": reads,
             "l2": "inputs larger than L2: every step streams the 1.55 GB packed genome and ~394 GB of FASTQ through the 126 MB L2"}
+
+
+class FastqSample:
+    """Sink of one read stage that keeps a fixed sample of the FASTQ it is handed: per file, WINDOWS windows of WIDTH bytes at
+    seeded offsets below the file's expected size. The offsets depend on the bench arguments only, so two builds sample the same
+    bytes. Window bytes past the end of a file stay -1."""
+    WINDOWS, WIDTH = 4096, 1024   # 2 files x 4096 x 1024 float32 = 32 MiB
+
+    def __init__(self, nfiles, expected_bytes, seed=0x5C55):
+        from scssim_b200 import api
+        self.offsets = np.sort(np.random.default_rng(seed).integers(0, max(int(expected_bytes), 1), self.WINDOWS))
+        self.data = [np.full((self.WINDOWS, self.WIDTH), -1.0, dtype=np.float32) for _ in range(nfiles)]
+        self.pos = [0] * nfiles
+        self.fn = api.SINK_FN(self._sink)
+
+    def _sink(self, _user, f, data, n):
+        lo, hi = self.pos[f], self.pos[f] + n
+        first, last = np.searchsorted(self.offsets, lo - self.WIDTH, side="right"), np.searchsorted(self.offsets, hi)
+        if last > first:
+            buf = np.ctypeslib.as_array(C.cast(data, C.POINTER(C.c_ubyte)), shape=(n,))
+            for k in range(first, last):
+                o = int(self.offsets[k])
+                a, b = max(o, lo), min(o + self.WIDTH, hi)
+                self.data[f][k, a - o:b - o] = buf[a - lo:b - lo]
+        self.pos[f] = hi
+        return 0
+
+    def save(self, d, stats):
+        """fastq_<file>.npy: (WINDOWS, WIDTH) bytes; fastq_offsets.npy: window offsets; fastq_bytes.npy: bytes per file, records."""
+        os.makedirs(d, exist_ok=True)
+        for f, arr in enumerate(self.data):
+            np.save(os.path.join(d, f"fastq_{f + 1}.npy"), arr)
+        np.save(os.path.join(d, "fastq_offsets.npy"), self.offsets.astype(np.float64))
+        np.save(os.path.join(d, "fastq_bytes.npy"), np.array(list(stats["fastq_bytes"]) + [stats["records"]], dtype=np.float64))
 
 
 class ClockSampler:
@@ -121,7 +162,7 @@ def measured_hbm_peak():
 
 # ------------------------------------------------------------------------------------------------ reference arm (CPU)
 def run_reference_cpu(tmp, profile, steps, warmup, coverage, sample_chrom=REF_SAMPLE_CHROM):
-    """The reference's own `scssim genreads -t <cores>` (compiled from /root/reference into oracle/_ref), one whole process per
+    """The reference's own `scssim genreads -t <cores>` (compiled into oracle/_ref by oracle/build_ref.sh), one whole process per
     step on the bounded sample cell. Stage times are taken from the moments its own stderr progress lines appear
     (Malbac.cpp:174,422,437; scssim.cpp:66). Returns a dict."""
     import helpers as H
@@ -192,9 +233,15 @@ def synth_chromosome_cuda(torch, length, seed, device, out_h1, out_h2):
         nsnp = int(n * SNP_RATE)
         pos = torch.randint(0, n, (nsnp,), generator=gen, device=device)
         shift = torch.randint(1, 4, (nsnp,), generator=gen, device=device, dtype=torch.uint8)
+        # a position drawn more than once takes its last draw, as numpy's assignment in synth.py does: a CUDA scatter with
+        # repeated indices leaves the winner undefined, which made the cell differ from run to run
+        pos, order = torch.sort(pos, stable=True)
+        last = torch.ones_like(pos, dtype=torch.bool)
+        last[:-1] = pos[1:] != pos[:-1]
+        pos, shift = pos[last], shift[order][last]
         code[pos] = (code[pos] + shift) & 3
         h2[lo:lo + n].copy_(lut[code.long()], non_blocking=False)
-        del idx, is_gc, pick, code, pos, shift
+        del idx, is_gc, pick, code, pos, shift, order, last
     torch.cuda.empty_cache()
 
 
@@ -283,7 +330,13 @@ def main():
     ap.add_argument("--slab-mb", type=int, default=64, help="FASTQ staging slab per file and buffer (MiB)")
     ap.add_argument("--files-dir", default=None, help="directory for the e2e_files leg (default: the system temp dir)")
     ap.add_argument("--gz", action="store_true", help="(not the headline) block-gzip output on the device: compressed FASTQ lands in the pinned ring")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of the FASTQ of the last timed step (rank 0's share) as DIR/<name>.npy (float32, float64)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     warmup = max(a.warmup, 0)
     # stdout carries exactly one JSON line: libraries that print there (NCCL's version banner) are sent to stderr
@@ -312,7 +365,6 @@ def main():
               "e2e": {"value": r["value"], "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}})
         return 0
 
-    import numpy as np
     import torch
     import torch.distributed as dist
     from scssim_b200 import api
@@ -438,13 +490,20 @@ def main():
                     weight = rate[rank]
                     g.set_shard_weight(weight)
                     weights_hist.append([round(x / sum(rate), 4) for x in rate])
+        sample = None
+        if a.dump_outputs and rank == 0:
+            # expected bytes of one of this rank's two files: its reads / 2 records of ~(header + bases + '+' + qualities) bytes
+            sample = FastqSample(2, config["reads_per_step"] / world / 2 * (2 * READ_LEN + 20))
         l0 = g.stats()["kernel_launches"]
         clocks = ClockSampler(device); clocks.start()
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         emit_ms = emit_n = reads_ms = amp_ms = alloc_ms = 0.0
         barrier(); ev0.record(); t0 = time.perf_counter()
-        for _ in range(a.steps):
-            step_resident()
+        for i in range(a.steps):
+            if sample and i == a.steps - 1:   # the last timed step hands its FASTQ to the sampling sink instead of discarding it
+                g.amplify().set_read_counts()._ck(api.lib().scs_yield_reads_sink(g._h, sample.fn, None))
+            else:
+                step_resident()
             st = g.stats()
             emit_ms += st["ms_emit_kernel"]; emit_n += st["emit_launches"]; reads_ms += st["ms_reads"]; amp_ms += st["ms_amplify"]; alloc_ms += st["ms_alloc"]
         ev1.record(); barrier(); wall = time.perf_counter() - t0
@@ -457,6 +516,8 @@ def main():
         fastq_bytes = st["fastq_bytes"][0] + st["fastq_bytes"][1]
         plain_bytes = st["plain_bytes"][0] + st["plain_bytes"][1]
         n_fulls, n_semis = st["n_fulls_global"], st["n_semis_global"]
+        if sample:
+            sample.save(a.dump_outputs, st)
 
         # ---- e2e leg (host buffers in, host bytes out); one untimed pass first (page faults of the host side)
         step_e2e()
@@ -569,7 +630,7 @@ def main():
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": a.gpus, "steps": a.steps, "warmup": a.warmup,
             "ms_per_step": dev_s / a.steps * 1e3, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "u8", "data": "synthetic",
             "config": config,
-            "detail": {"reads_per_step": reads_all, "fastq_bytes_per_step": bytes_all, "fastq_GBps": gbps, "gzip": bool(a.gz), "plain_bytes_per_step_rank0": plain_bytes, "full_amplicons": n_fulls, "semi_amplicons": n_semis,
+            "detail": {"dump_outputs": sample is not None, "reads_per_step": reads_all, "fastq_bytes_per_step": bytes_all, "fastq_GBps": gbps, "gzip": bool(a.gz), "plain_bytes_per_step_rank0": plain_bytes, "full_amplicons": n_fulls, "semi_amplicons": n_semis,
                        "stage_ms_per_step_rank0": {"amplify": amp_ms / a.steps, "alloc": alloc_ms / a.steps, "reads": reads_ms / a.steps},
                        "reads_stage_ms_max_rank": reads_ms_max / a.steps,
                        "parallelism": (f"one cell over {world} GPUs: sequences sharded for the amplification, packed genome + amplicon table all-gathered "

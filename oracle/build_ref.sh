@@ -1,22 +1,23 @@
 #!/usr/bin/env bash
-# TEST INFRASTRUCTURE. Builds the reference's own C++ (read where it lies under
-# /root/reference) into oracle/_ref/ — two binaries:
+# TEST INFRASTRUCTURE. Builds the reference's own C++ (the original SCSsim
+# sources, read at BASELINE.json's reference_path, or where $SCS_REFERENCE_DIR
+# points when it is set) into oracle/_ref/ — two binaries:
 #   oracle/_ref/bin/scssim         the reference + the five missing `return`s
 #                                  (SURVEY.md §8c: without them g++ >= 8 emits
 #                                  code that crashes); behaviour otherwise stock.
 #   oracle/_ref/bin/scssim_replay  same + seed from $SCS_SEED and a log of every
 #                                  random draw to $SCS_REPLAY_LOG.* (ref_hooks.h).
-# Nothing from /root/reference is committed: the patched copies live only under
+# Nothing from the reference is committed: the patched copies live only under
 # the git-ignored oracle/_ref/src. Uses g++ directly (no cmake).
 set -euo pipefail
 HERE="$(cd "$(dirname "${BASH_SOURCE[0]}")" && pwd)"
-REF="${SCS_REFERENCE_DIR:-/root/reference}"
+REF="${SCS_REFERENCE_DIR-$(python3 -c 'import json, sys; print(json.load(open(sys.argv[1])).get("reference_path", ""))' "$HERE/../BASELINE.json")}"
 OUT="$HERE/_ref"
-if [ ! -d "$REF/lib" ]; then
+if [ -z "$REF" ] || [ ! -d "$REF/lib" ]; then
     if [ -x "$OUT/bin/scssim" ] && [ -x "$OUT/bin/scssim_replay" ]; then
-        echo "build_ref: $REF absent, keeping prebuilt $OUT/bin" >&2; exit 0
+        echo "build_ref: no SCSsim sources at '$REF', keeping prebuilt $OUT/bin" >&2; exit 0
     fi
-    echo "build_ref: $REF absent and no prebuilt binaries" >&2; exit 1
+    echo "build_ref: no SCSsim sources at '$REF' and no prebuilt binaries" >&2; exit 1
 fi
 if [ -x "$OUT/bin/scssim" ] && [ -x "$OUT/bin/scssim_replay" ] && \
    [ "$OUT/bin/scssim_replay" -nt "$HERE/ref_hooks.cpp" ] && [ "$OUT/bin/scssim_replay" -nt "$HERE/build_ref.sh" ]; then

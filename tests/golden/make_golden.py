@@ -1,6 +1,6 @@
 """Regenerates tests/golden/replay_pe2500 by running the reference itself (oracle/_ref/bin/scssim_replay,
-built from /root/reference by oracle/build_ref.sh) in THIS container. Committed so the fixture's origin
-is reproducible:  python tests/golden/make_golden.py
+built by oracle/build_ref.sh from the SCSsim sources at BASELINE.json's reference_path, or at $SCS_REFERENCE_DIR
+when set). Committed so the fixture's origin is reproducible:  python tests/golden/make_golden.py
 """
 import lzma
 import os

@@ -1,6 +1,6 @@
 """Generates tests/golden/simuvars_small/: random inputs + the output of the REFERENCE binary itself
-(oracle/_ref/bin/scssim simuvars, built from /root/reference by oracle/build_ref.sh). Run in the build container:
-    python tests/golden/make_simuvars_golden.py
+(oracle/_ref/bin/scssim simuvars, built by oracle/build_ref.sh from the SCSsim sources at BASELINE.json's reference_path,
+or at $SCS_REFERENCE_DIR when set):  python tests/golden/make_simuvars_golden.py
 """
 import hashlib
 import json

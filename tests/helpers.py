@@ -5,10 +5,12 @@ Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline leg may touch o
 """
 import ctypes as C
 import functools
+import json
 import lzma
 import os
 import subprocess
 import sys
+import tempfile
 
 import numpy as np
 
@@ -20,9 +22,20 @@ ORACLE_DIR = os.path.join(ROOT, "oracle")
 PROFILES = ["Illumina_HiSeq2500", "Illumina_HiSeqXTen", "Illumina_HiSeq2000", "Illumina_GenomeAnalyzerIIx"]
 
 
+def reference_dir() -> str:
+    """Where the original SCSsim sources (lib/, src/) lie, which oracle/build_ref.sh compiles into oracle/_ref: the
+    reference_path that BASELINE.json declares, or SCS_REFERENCE_DIR when set. They are not part of this repository."""
+    d = os.environ.get("SCS_REFERENCE_DIR")
+    if d is None:
+        with open(os.path.join(ROOT, "BASELINE.json")) as f:
+            d = json.load(f).get("reference_path", "")
+    return d
+
+
 @functools.lru_cache(maxsize=None)
 def scratch_dir() -> str:
-    d = os.environ.get("SCS_TEST_SCRATCH", "/tmp/scssim_b200_tests")
+    # per user: on a shared machine another user's directory of the same name is not writable
+    d = os.environ.get("SCS_TEST_SCRATCH") or os.path.join(tempfile.gettempdir(), f"scssim_b200_tests_{os.getuid()}")
     os.makedirs(d, exist_ok=True)
     return d
 
@@ -65,13 +78,23 @@ def oracle_lib():
     return L
 
 
+def have_reference_sources() -> bool:
+    d = reference_dir()
+    return bool(d) and os.path.isdir(os.path.join(d, "lib"))
+
+
+def build_reference():
+    """oracle/build_ref.sh on the sources of reference_dir() (a no-op when the binaries are up to date)."""
+    subprocess.run(["bash", os.path.join(ORACLE_DIR, "build_ref.sh")], check=True, env=dict(os.environ, SCS_REFERENCE_DIR=reference_dir()))
+
+
 def ref_replay_bin():
     """The compiled reference with seed/draw-log hooks (oracle/build_ref.sh); None if it was never built."""
     p = os.path.join(ORACLE_DIR, "_ref", "bin", "scssim_replay")
     if os.path.exists(p):
         return p
-    if os.path.isdir("/root/reference/lib"):
-        subprocess.run(["bash", os.path.join(ORACLE_DIR, "build_ref.sh")], check=True)
+    if have_reference_sources():
+        build_reference()
         return p if os.path.exists(p) else None
     return None
 
@@ -184,8 +207,8 @@ def ref_bin():
     p = os.path.join(ORACLE_DIR, "_ref", "bin", "scssim")
     if os.path.exists(p):
         return p
-    if os.path.isdir("/root/reference/lib"):
-        subprocess.run(["bash", os.path.join(ORACLE_DIR, "build_ref.sh")], check=True)
+    if have_reference_sources():
+        build_reference()
         return p if os.path.exists(p) else None
     return None
 

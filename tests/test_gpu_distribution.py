@@ -108,7 +108,7 @@ def test_free_running_matches_reference_distributions(tmp_path):
     from scssim_b200 import api
     exe = H.ref_replay_bin()   # the seedable build: both sides of this test are then deterministic
     if exe is None:
-        pytest.skip("compiled reference (oracle/_ref) not on this box")
+        pytest.skip("needs the original SCSsim sources at BASELINE.json's reference_path or SCS_REFERENCE_DIR")
     tmp = str(tmp_path)
     fa = os.path.join(tmp, "cell.fa")
     genome = H.write_genome(fa, 1, 600_000, seed=23)

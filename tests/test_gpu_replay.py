@@ -5,8 +5,8 @@ are fed to the CUDA path, which must then write the reference's FASTQ byte for b
   CPU oracle in tape mode                                   -> FASTQ_orc (== FASTQ_ref) + per-entity tape offsets
   CUDA path with the tapes + offsets                        -> FASTQ_gpu  == FASTQ_ref
 
-The reference binary travels to the GPU box prebuilt (oracle/_ref is git-ignored, not gpurun-ignored);
-the committed golden case below covers boxes where it is absent.
+The live cases build the reference from the SCSsim sources at BASELINE.json's reference_path (or SCS_REFERENCE_DIR; or use a prebuilt,
+git-ignored oracle/_ref) and skip without them; the committed golden case below needs neither.
 """
 import os
 
@@ -44,7 +44,7 @@ def _replay_case(tmp, fa, profile, layout, gamma, coverage, isize, tape_prefix, 
 ])
 def test_replay_against_live_reference(tmp_path, profile, layout, gamma, coverage, isize, glen):
     if H.ref_replay_bin() is None:
-        pytest.skip("oracle/_ref/bin/scssim_replay not built on this box")
+        pytest.skip("needs the original SCSsim sources at BASELINE.json's reference_path or SCS_REFERENCE_DIR")
     tmp = str(tmp_path)
     fa = os.path.join(tmp, "cell.fa")
     H.write_genome(fa, 1, glen, seed=11)

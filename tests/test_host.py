@@ -293,3 +293,26 @@ def test_bench_reference_arm_contract():
         assert set(d["cpu_baseline"]["stage_s"]) == {"load_frags", "amplify", "alloc", "reads"} and d["cpu_baseline"]["reads_stage_value"] > 0
     assert d["cpu_baseline"]["kind"] in ("reference", "port") and d["cpu_baseline"]["cores"] >= 1
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+
+
+def test_bench_fastq_sample_windows_hold_the_bytes_at_their_offsets():
+    """bench.py --dump-outputs: the sink, fed a known byte stream per file in uneven slabs through its ctypes entry point as the
+    library calls it, keeps in every window exactly the bytes at the window's offset; bytes past the end of a file stay -1."""
+    import bench
+    rng = np.random.default_rng(3)
+    streams = [rng.integers(0, 256, 5_000_000, dtype=np.uint8), rng.integers(0, 256, 1_234_567, dtype=np.uint8)]
+    s = bench.FastqSample(2, 4_000_000)
+    for f, st in enumerate(streams):
+        p = 0
+        while p < len(st):
+            chunk = np.ascontiguousarray(st[p:p + int(rng.integers(1, 300_000))])
+            assert s.fn(None, f, chunk.ctypes.data, len(chunk)) == 0
+            p += len(chunk)
+    for f, st in enumerate(streams):
+        assert s.pos[f] == len(st)
+        for k, o in enumerate(s.offsets):
+            want = np.full(s.WIDTH, -1.0, dtype=np.float32)
+            seg = st[o:o + s.WIDTH]
+            want[:len(seg)] = seg
+            assert np.array_equal(s.data[f][k], want), (f, k, o)
+    assert (s.offsets + s.WIDTH > len(streams[1])).sum() > 1000   # file 2 ends inside the sampled range

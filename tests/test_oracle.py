@@ -46,7 +46,7 @@ LIVE = [
 @pytest.mark.parametrize("profile,layout,gamma,coverage,isize,nchrom,glen", LIVE)
 def test_oracle_reproduces_live_reference(tmp_path, profile, layout, gamma, coverage, isize, nchrom, glen):
     if H.ref_replay_bin() is None:
-        pytest.skip("reference not built (no /root/reference on this box)")
+        pytest.skip("needs the original SCSsim sources at BASELINE.json's reference_path or SCS_REFERENCE_DIR")
     tmp = str(tmp_path)
     fa = os.path.join(tmp, "cell.fa")
     H.write_genome(fa, nchrom, glen, seed=3, width=60)
