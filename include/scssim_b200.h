@@ -66,6 +66,13 @@ typedef struct scs_params {
     int32_t relay_device; /* -1 (default): FASTQ slabs are copied to the host over this GPU's own link. >= 0: over NVLink to that peer
                              GPU first and from there to the host — for boxes where some GPUs sit behind a slow or shared host link
                              (bench.py measures the links and lets the GPUs of the slow group relay through the fast group) */
+    int32_t host_expand;  /* FASTQ slabs sent as packed base+quality records and expanded into text by host threads, so that the host link
+                             carries ~47 % fewer bytes for them. -1 (default, auto): for every slab the read stage picks whichever path,
+                             text over the link or packed + host expansion, is estimated to finish sooner (moving averages of the link
+                             rate and of the expansion rate); on only for world = 1, gzip = 0 and scs_yield_reads_sink. 0: off.
+                             1: every slab packed; 2: every other slab packed (1 and 2 also at world > 1; both for tests). The bytes
+                             a sink receives are the same FASTQ text on every path; scs_yield_reads (files) always sends text */
+    int32_t expand_threads; /* host threads of the expansion pool; 0 -> default (CPUs in the process's affinity mask - 1) */
 } scs_params;
 
 void scs_default_params(scs_params* p);
@@ -143,6 +150,8 @@ typedef struct scs_stats {
     uint64_t emit_launches;
     uint64_t genome_window_bytes;              /* algorithmic HBM read bytes of the emit kernel */
     uint64_t plain_bytes[2];                   /* FASTQ text bytes behind fastq_bytes (equal unless gzip = 1, then fastq_bytes is compressed) */
+    uint64_t link_bytes[2];                    /* bytes that crossed the host link per file (packed slabs: records + split table) */
+    uint64_t slabs_packed, slabs;              /* slabs sent packed (host_expand) / all slabs of the last read stage */
 } scs_stats;
 int scs_get_stats(const scs_ctx* ctx, scs_stats* out);
 
@@ -210,6 +219,11 @@ int scs_test_async_writer(const char* path, const char* data, uint64_t n, uint64
 int scs_test_deflate_code(const scs_ctx* ctx, uint8_t* lens257, uint32_t* prefix_words, int cap_words, uint32_t* prefix_bits);
 /* The first n values of libc rand() after srand(seed), as reproduced by the library. */
 int scs_test_libc_rand(uint32_t seed, int n, uint32_t* out);
+/* Host-only: the expansion pool of host_expand on one packed slab without a GPU. `wire` is the slab as it leaves the device: nsplit
+ * split entries (u64 wire offset, u64 text offset of every 2048th record slot), then wire_bytes bytes of records (wire.h).
+ * Writes text_bytes bytes of FASTQ to out with `threads` threads; qchar0 = '!' + the profile's lowest quality index;
+ * scalar != 0 forces the scalar expander. Returns 0, or SCS_E_ARG when the slab is malformed. */
+int scs_test_expand_wire(const uint8_t* wire, uint32_t nsplit, uint64_t wire_bytes, uint64_t text_bytes, int qchar0, int threads, int scalar, char* out);
 
 /* ---- replay ("recorded draws", BASELINE north_star correctness part 1) -------------------------
  * Tapes are the u32 logs of the patched reference run with -t 1; marks give, per entity, the tape

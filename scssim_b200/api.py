@@ -35,7 +35,8 @@ class Params(C.Structure):
     _fields_ = [("primers", C.c_int64), ("gamma", C.c_double), ("coverage", C.c_double), ("isize", C.c_int32),
                 ("paired", C.c_int32), ("seed", C.c_uint64), ("device", C.c_int32), ("rank", C.c_int32),
                 ("world", C.c_int32), ("balance", C.c_int32), ("slab_bytes", C.c_uint64), ("io_threads", C.c_int32),
-                ("ring_slabs", C.c_int32), ("gzip", C.c_int32), ("relay_device", C.c_int32)]
+                ("ring_slabs", C.c_int32), ("gzip", C.c_int32), ("relay_device", C.c_int32), ("host_expand", C.c_int32),
+                ("expand_threads", C.c_int32)]
 
 
 class Stats(C.Structure):
@@ -45,13 +46,14 @@ class Stats(C.Structure):
                 ("total_primers_left", C.c_uint64), ("kernel_launches", C.c_uint64), ("ms_pack", C.c_double),
                 ("ms_amplify", C.c_double), ("ms_alloc", C.c_double), ("ms_reads", C.c_double),
                 ("ms_reads_kernels", C.c_double), ("ms_emit_kernel", C.c_double), ("emit_launches", C.c_uint64),
-                ("genome_window_bytes", C.c_uint64), ("plain_bytes", C.c_uint64 * 2)]
+                ("genome_window_bytes", C.c_uint64), ("plain_bytes", C.c_uint64 * 2), ("link_bytes", C.c_uint64 * 2),
+                ("slabs_packed", C.c_uint64), ("slabs", C.c_uint64)]
 
     def as_dict(self):
         d = {}
         for name, _ in self._fields_:
             v = getattr(self, name)
-            d[name] = list(v) if name in ("fastq_bytes", "plain_bytes") else v
+            d[name] = list(v) if name in ("fastq_bytes", "plain_bytes", "link_bytes") else v
         return d
 
 
@@ -88,7 +90,8 @@ EXPORTS = ["scs_default_params", "scs_create", "scs_destroy", "scs_last_error", 
            "scs_test_predict", "scs_test_philox", "scs_test_det_log", "scs_profile_thresholds", "scs_shard_range",
            "scs_version", "scs_device_count", "scs_nccl_unique_id", "scs_nccl_init", "scs_nccl_abort", "scs_nccl_version",
            "scs_simuvars_default_params", "scs_simuvars", "scs_simuvars_sink", "scs_simuvars_to_genome", "scs_simuvars_get_stats",
-           "scs_simuvars_warnings", "scs_svplan_create", "scs_svplan_destroy", "scs_svplan_dump", "scs_test_libc_rand", "scs_shard_sequences", "scs_test_fasta_index", "scs_test_file_writer", "scs_test_async_writer", "scs_test_deflate_code"]
+           "scs_simuvars_warnings", "scs_svplan_create", "scs_svplan_destroy", "scs_svplan_dump", "scs_test_libc_rand", "scs_shard_sequences", "scs_test_fasta_index", "scs_test_file_writer", "scs_test_async_writer", "scs_test_deflate_code",
+           "scs_test_expand_wire"]
 
 _lib = None
 
@@ -191,6 +194,17 @@ def write_file_parallel(path: str, data: bytes, slab_bytes: int, threads: int) -
         raise ScsError(rc, f"can not write {path}")
 
 
+def expand_wire(wire: bytes, nsplit: int, text_bytes: int, qchar0: int = 33, threads: int = 1, scalar: bool = False) -> bytes:
+    """Expand one packed FASTQ slab (scssim_b200/csrc/wire.h: nsplit 16-byte split entries, then the records) with the host
+    expansion pool of host_expand (host only). Returns the text_bytes bytes of FASTQ."""
+    out = C.create_string_buffer(max(int(text_bytes), 1))
+    lib().scs_test_expand_wire.argtypes = [C.c_char_p, C.c_uint32, C.c_uint64, C.c_uint64, C.c_int, C.c_int, C.c_int, C.c_void_p]
+    rc = lib().scs_test_expand_wire(wire, nsplit, len(wire) - 16 * nsplit, text_bytes, qchar0, threads, int(scalar), out)
+    if rc != SCS_OK:
+        raise ScsError(rc, "malformed packed slab")
+    return out.raw[:text_bytes]
+
+
 def write_file_async(path: str, data: bytes, slab_bytes: int, threads: int = 4, ring: int = 4, base: int = 0, create: bool = True, prealloc: int = 0,
                      direct: bool = True) -> bool:
     """Feed `data` through the asynchronous file sink of scs_yield_reads (host only). Returns whether O_DIRECT was in use."""
@@ -232,7 +246,8 @@ class GenReads:
 
     def __init__(self, primers: int = 100000, gamma: float = 1e-9, coverage: float = 5.0, isize: int = 260,
                  layout: str = "PE", seed: int = 0x5C55, device: int = 0, rank: int = 0, world: int = 1,
-                 slab_bytes: int = 0, balance: bool = False, io_threads: int = 0, ring_slabs: int = 0, gzip: bool = False, relay_device: int = -1):
+                 slab_bytes: int = 0, balance: bool = False, io_threads: int = 0, ring_slabs: int = 0, gzip: bool = False, relay_device: int = -1,
+                 host_expand: int = -1, expand_threads: int = 0):
         if layout not in ("SE", "PE"):
             raise ScsError(SCS_E_ARG, "Error: sequence layout incorrectly specified!\nshould be SE (single end) or PE (paired-end)")
         L = lib()
@@ -245,6 +260,8 @@ class GenReads:
         p.ring_slabs = ring_slabs
         p.gzip = int(gzip)
         p.relay_device = relay_device
+        p.host_expand = host_expand
+        p.expand_threads = expand_threads
         self._h = C.c_void_p()
         rc = L.scs_create(C.byref(p), C.byref(self._h))
         if rc != SCS_OK:

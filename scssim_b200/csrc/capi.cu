@@ -9,6 +9,7 @@
 #include "slab_sink.h"
 #include "simuvars_plan.h"
 #include "deflate_host.h"
+#include "expand_host.h"
 
 using namespace scs;
 
@@ -24,6 +25,7 @@ void scs_default_params(scs_params* p) {
     memset(p, 0, sizeof(*p));
     p->primers = 100000; p->gamma = 1e-9; p->coverage = 5; p->isize = 260; p->paired = 1;   // src/scssim.cpp:289-293
     p->seed = 0x5C55ull; p->device = 0; p->rank = 0; p->world = 1; p->balance = 0; p->slab_bytes = 0; p->io_threads = 0; p->ring_slabs = 0; p->gzip = 0; p->relay_device = -1;
+    p->host_expand = -1; p->expand_threads = 0;
 }
 
 int scs_create(const scs_params* p, scs_ctx** out) {
@@ -59,6 +61,7 @@ void scs_destroy(scs_ctx* c) {
     if (!c) return;
     const bool dev = c->have_device;
     cudaStream_t st = c->st, st_copy = c->st_copy;
+    delete c->pool; c->pool = nullptr;   // joins the expansion threads (no job is in flight between calls)
     if (dev) {
         cudaSetDevice(c->P.device); alloc_stream() = c->st;
         cudaDeviceSynchronize();
@@ -70,6 +73,7 @@ void scs_destroy(scs_ctx* c) {
             cudaSetDevice(c->P.device);
         }
         for (int f = 0; f < 2; f++) for (char* q : c->ring_host[f]) cudaFreeHost(q);
+        for (int f = 0; f < 2; f++) for (char* q : c->wire_host[f]) cudaFreeHost(q);
         if (c->rscratch.htotals) cudaFreeHost(c->rscratch.htotals);
         for (int b = 0; b < 2; b++) if (c->sv_pinned[b]) cudaFreeHost(c->sv_pinned[b]);
     }
@@ -355,6 +359,16 @@ int scs_test_deflate_code(const scs_ctx* c, uint8_t* lens, uint32_t* prefix_word
     if (prefix_words) { if (cap_words < nw) return SCS_E_ARG; memcpy(prefix_words, D.prefix_words.data(), (size_t)nw * 4); }
     return nw;
 }
+int scs_test_expand_wire(const uint8_t* wire, uint32_t nsplit, uint64_t wire_bytes, uint64_t text_bytes, int qchar0, int threads, int scalar, char* out) {
+    if ((!wire && (nsplit || wire_bytes)) || (!out && text_bytes) || threads < 1) return SCS_E_ARG;
+    ExpandPool pool(-1, threads);
+    ExpandJob j;
+    j.wire[0] = wire; j.nsplit[0] = nsplit; j.wire_bytes[0] = wire_bytes; j.text_bytes[0] = text_bytes; j.out[0] = out;
+    j.qchar0 = qchar0; j.scalar = scalar != 0;
+    pool.submit(&j);
+    return pool.wait(&j) ? SCS_E_ARG : SCS_OK;
+}
+
 int scs_test_libc_rand(uint32_t seed, int n, uint32_t* out) {
     if (!out || n < 0) return SCS_E_ARG;
     sv::LibcRand r(seed);

@@ -160,7 +160,8 @@ struct ReadScratch {
     DevBuf<uint64_t> off1, off2, scan, totals;
     DevBuf<int> flags; DevBuf<unsigned long long> records;
     DevBuf<char> stage[2];         // fixed-stride records of one slab per file (staged emit), packed by compact_records_kernel
-    uint64_t* htotals = nullptr;   // pinned + mapped
+    DevBuf<uint32_t> wsize[2]; DevBuf<uint64_t> woff[2];   // packed slabs (wire.h): wire bytes per record and their scan
+    uint64_t* htotals = nullptr;   // pinned + mapped: [2b + f] bytes of buffer b, file f; [4 + ...] gzip text; [8 + ...] wire records
     uint64_t* dtotals_mapped = nullptr;   // device view of htotals
 };
 
@@ -174,6 +175,8 @@ struct GzState {
 };
 
 }  // namespace scs
+
+namespace scs { class ExpandPool; }
 
 struct scs_ctx {
     scs_params P;
@@ -238,6 +241,11 @@ struct scs_ctx {
     scs::DevBuf<char> slab_dev[2][2];   // [buffer][file] packed device slabs
     std::vector<char*> ring_host[2];    // [file] ring of pinned host slots the slabs are copied into (slab_sink.h)
     uint64_t slab_cap = 0;
+    // packed slabs (host_expand): pinned wire slots the packed slabs land in, the threads that expand them, the profile's lowest
+    // quality index (a packed quality is q - wire_qlo)
+    std::vector<char*> wire_host[2]; uint64_t wire_cap = 0;
+    scs::ExpandPool* pool = nullptr;
+    uint32_t wire_qlo = 0;
 
     int fail(int code, const std::string& msg) { err = msg; return code; }
 };

@@ -18,9 +18,13 @@
 #include <cstdlib>
 #include <cstring>
 
+#include <sched.h>
+
 #define SCS_PHILOX_OUTLINE 1
 #include "ctx.h"
+#include "expand_host.h"
 #include "slab_sink.h"
+#include "wire.h"
 
 namespace scs {
 
@@ -767,6 +771,70 @@ __global__ void __launch_bounds__(256) compact_records_kernel(const char* __rest
     }
 }
 
+// ---- packed slabs (wire.h). A staged record packs unless it holds a base outside ACGT or a quality outside [qlo, qlo + 63];
+// ---- the warp reads it once to decide, and returns its header length.
+__device__ __forceinline__ bool record_packs(const uint8_t* __restrict__ src, int sz, uint32_t qlo, int lane, int* hl_out) {
+    const uint32_t nl = __ballot_sync(0xffffffffu, lane < sz && src[lane] == '\n');
+    const int hl = nl ? __ffs(nl) : 0;
+    *hl_out = hl;
+    const int np = (sz - hl - 4) / 2;
+    if (!hl || hl >= wire::kVerbatim || np < 0 || hl + 2 * np + 4 != sz) return false;
+    bool ok = true;
+    for (int k = lane; k < np; k += 32) {
+        const uint8_t b = src[hl + k];
+        const uint32_t q = (uint32_t)src[hl + np + 3 + k] - 33u - qlo;
+        ok &= (b == 'A' || b == 'C' || b == 'G' || b == 'T') && q < (uint32_t)wire::kQualSpan;
+    }
+    return __all_sync(0xffffffffu, ok);
+}
+
+__global__ void __launch_bounds__(256) wire_size_kernel(const char* __restrict__ stage, uint64_t stride, const uint32_t* __restrict__ sizes, uint64_t n,
+                                                        uint32_t qlo, uint32_t* __restrict__ wsizes) {
+    const int lane = threadIdx.x & 31;
+    for (uint64_t ls = (uint64_t)blockIdx.x * 8 + (threadIdx.x >> 5); ls < n; ls += (uint64_t)gridDim.x * 8) {
+        const int sz = (int)sizes[ls];
+        uint32_t w = 0;
+        if (sz) {
+            int hl;
+            const bool pk = record_packs(reinterpret_cast<const uint8_t*>(stage) + ls * stride, sz, qlo, lane, &hl);
+            w = pk ? wire::packed_bytes(hl, (sz - hl - 4) / 2) : 3u + (uint32_t)sz;
+        }
+        if (lane == 0) wsizes[ls] = w;
+    }
+}
+
+// the packed slab of one file: the split table (one {wire, text} offset pair per kSplitEvery slots) at `out`, the records after it
+__global__ void __launch_bounds__(256) pack_records_kernel(const char* __restrict__ stage, uint64_t stride, const uint32_t* __restrict__ sizes,
+                                                           const uint64_t* __restrict__ toffs, const uint64_t* __restrict__ woffs, uint64_t n, uint32_t qlo,
+                                                           char* __restrict__ out, uint64_t cap, int* __restrict__ flags) {
+    const int lane = threadIdx.x & 31;
+    const uint64_t nsplit = (n + wire::kSplitEvery - 1) / wire::kSplitEvery;
+    wire::Split* split = reinterpret_cast<wire::Split*>(out);
+    uint8_t* rec0 = reinterpret_cast<uint8_t*>(out) + nsplit * sizeof(wire::Split);
+    for (uint64_t ls = (uint64_t)blockIdx.x * 8 + (threadIdx.x >> 5); ls < n; ls += (uint64_t)gridDim.x * 8) {
+        if (lane == 0 && ls % wire::kSplitEvery == 0) split[ls / wire::kSplitEvery] = wire::Split{woffs[ls], toffs[ls]};
+        const int sz = (int)sizes[ls];
+        if (!sz) continue;
+        const uint8_t* src = reinterpret_cast<const uint8_t*>(stage) + ls * stride;
+        int hl;
+        const bool pk = record_packs(src, sz, qlo, lane, &hl);
+        const int np = (sz - hl - 4) / 2;
+        const uint32_t wsz = pk ? wire::packed_bytes(hl, np) : 3u + (uint32_t)sz;
+        const uint64_t o = woffs[ls];
+        if (nsplit * sizeof(wire::Split) + o + wsz > cap) { if (lane == 0) atomicOr(flags, 16); continue; }
+        uint8_t* dst = rec0 + o;
+        const uint32_t len = pk ? (uint32_t)np : (uint32_t)sz;
+        if (lane == 0) { dst[0] = pk ? (uint8_t)hl : (uint8_t)wire::kVerbatim; dst[1] = (uint8_t)(len & 255u); dst[2] = (uint8_t)(len >> 8); }
+        if (!pk) { for (int k = lane; k < sz; k += 32) dst[3 + k] = src[k]; continue; }
+        for (int k = lane; k < hl; k += 32) dst[3 + k] = src[k];
+        for (int k = lane; k < np; k += 32) {
+            const uint8_t b = src[hl + k];
+            const uint32_t code = b == 'A' ? 0u : b == 'C' ? 1u : b == 'G' ? 2u : 3u;
+            dst[3 + hl + k] = (uint8_t)(code | (((uint32_t)src[hl + np + 3 + k] - 33u - qlo) << 2));
+        }
+    }
+}
+
 // ---- slow path (insert sizes that can exceed an amplicon, -s large): failed attempts per slot -----
 __global__ void __launch_bounds__(256) fail_count_kernel(DrawSrc dsrc, ReadTables T, SlabArgs A, uint32_t* __restrict__ nfail) {
     uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -825,6 +893,8 @@ int upload_profile(scs_ctx* c) {
         meta[o] = (uint32_t)lo | ((uint32_t)cnt << 8);
     }
     SCS_CUDA(c, up32(D.qualDiag, rows)); SCS_CUDA(c, up32(D.qualDiagPiv, piv)); SCS_CUDA(c, up32(D.qualDiagMeta, meta));
+    // packed slabs: the lowest quality index any row can produce (a draw counts at least the row's leading zero thresholds)
+    c->wire_qlo = P.qualLo.empty() ? 0u : (uint32_t)*std::min_element(P.qualLo.begin(), P.qualLo.end());
     return SCS_OK;
 }
 
@@ -853,8 +923,8 @@ static ReadTables make_tables(const scs_ctx* c) {
 // ---------------------------------------------------------------------------------- slab pipeline
 namespace {
 
-// events of one run of the stage; every exit path (errors included) first drains both streams, so nothing that was queued
-// can still touch the context's buffers when the caller retries
+// events of one run of the stage; every exit path (errors included) first drains both streams and the expansion pool, so
+// nothing that was queued can still touch the context's buffers or these events when the caller retries
 struct StageGuard {
     scs_ctx* c; std::vector<cudaEvent_t> evs;
     explicit StageGuard(scs_ctx* ctx) : c(ctx) {}
@@ -862,22 +932,28 @@ struct StageGuard {
     ~StageGuard() {
         cudaStreamSynchronize(c->st); cudaStreamSynchronize(c->st_copy);
         if (c->st_relay) cudaStreamSynchronize(c->st_relay);
+        if (c->pool) c->pool->drain();
         for (cudaEvent_t e : evs) if (e) cudaEventDestroy(e);
     }
 };
 
 }  // namespace
 
-// scs_sink_fn adapter: two ring slots, the user's function runs on the launching thread in slab order
+// scs_sink_fn adapter: kSlots ring slots, the user's function runs on the launching thread in slab order
 CallbackConsumer::CallbackConsumer(scs_sink_fn f, void* u) : fn(f), user(u) {}
 int CallbackConsumer::consume_front(bool wait) {
     if (count == 0) return 0;
     Pending& q = pend[head];
-    if (wait) { if (cudaEventSynchronize(q.ev) != cudaSuccess) return 1; }
+    if (q.job) {   // text written by the expansion pool
+        if (wait) { if (q.pool->wait(q.job)) return 1; }
+        else if (!q.pool->query(q.job)) return -1;
+        else if (q.pool->wait(q.job)) return 1;
+    }
+    else if (wait) { if (cudaEventSynchronize(q.ev) != cudaSuccess) return 1; }
     else if (cudaEventQuery(q.ev) != cudaSuccess) { (void)cudaGetLastError(); return -1; }   // not landed yet
     int rc = 0;
     if (fn) for (int f = 0; f < 2 && !rc; f++) if (q.n[f]) rc = fn(user, f, q.p[f], q.n[f]) ? 1 : 0;
-    q.live = false; head ^= 1; count--;
+    q.live = false; head = (head + 1) % kSlots; count--;
     return rc;
 }
 int CallbackConsumer::acquire(int slot) {
@@ -886,9 +962,14 @@ int CallbackConsumer::acquire(int slot) {
 }
 int CallbackConsumer::submit(int slot, cudaEvent_t copied, char* const p[2], const uint64_t bytes[2]) {
     Pending& q = pend[slot];
-    q.live = true; q.ev = copied; q.p[0] = p[0]; q.p[1] = p[1]; q.n[0] = bytes[0]; q.n[1] = bytes[1];
+    q.live = true; q.ev = copied; q.pool = nullptr; q.job = nullptr; q.p[0] = p[0]; q.p[1] = p[1]; q.n[0] = bytes[0]; q.n[1] = bytes[1];
     if (count == 0) head = slot;
     count++;
+    return 0;
+}
+int CallbackConsumer::submit_expanded(int slot, ExpandPool* pool, ExpandJob* job, char* const p[2], const uint64_t bytes[2]) {
+    if (submit(slot, nullptr, p, bytes)) return 1;
+    pend[slot].pool = pool; pend[slot].job = job;
     return 0;
 }
 int CallbackConsumer::service() {
@@ -951,10 +1032,11 @@ static int prepare_read_run(scs_ctx* c, ReadRun& R) {
     SCS_CUDA(c, W.flags.reserve(1)); SCS_CUDA(c, W.records.reserve(1)); SCS_CUDA(c, W.totals.reserve(4));
     SCS_CUDA(c, W.size1.reserve(R.batch + 1)); SCS_CUDA(c, W.size2.reserve(R.batch + 1));
     SCS_CUDA(c, W.off1.reserve(R.batch + 1)); SCS_CUDA(c, W.off2.reserve(R.batch + 1)); SCS_CUDA(c, W.scan.reserve(2 * 2048 + 16));
+    for (int f = 0; f < 2; f++) { SCS_CUDA(c, W.wsize[f].reserve(R.batch + 1)); SCS_CUDA(c, W.woff[f].reserve(R.batch + 1)); }
     // slab byte totals are written by the scan kernel straight into mapped pinned memory: a D2H memcpy on the compute
     // stream would queue behind the previous slab's 0.5 GB copy on the same copy engine and stall the emit kernel
     if (!W.htotals) {
-        SCS_CUDA(c, cudaHostAlloc((void**)&W.htotals, 64, cudaHostAllocMapped));
+        SCS_CUDA(c, cudaHostAlloc((void**)&W.htotals, 128, cudaHostAllocMapped));
         SCS_CUDA(c, cudaHostGetDevicePointer((void**)&W.dtotals_mapped, W.htotals, 0));
     }
     int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&R.sms, cudaDevAttrMultiProcessorCount, dev);
@@ -1033,6 +1115,7 @@ int yield_reads(scs_ctx* c, SlabConsumer& sink) {
     if (int rc = prepare_read_run(c, R)) return rc;
     c->stats.records = 0; c->stats.fastq_bytes[0] = c->stats.fastq_bytes[1] = 0; c->stats.plain_bytes[0] = c->stats.plain_bytes[1] = 0;
     c->stats.ms_reads = c->stats.ms_reads_kernels = c->stats.ms_emit_kernel = 0; c->stats.emit_launches = 0; c->stats.genome_window_bytes = 0;
+    c->stats.link_bytes[0] = c->stats.link_bytes[1] = 0; c->stats.slabs_packed = c->stats.slabs = 0;
     const bool gz = c->P.gzip != 0;
     if (R.nslots == 0 && !gz) return sink.finish() ? c->fail(SCS_E_IO, "FASTQ sink failed") : SCS_OK;
     if (gz) { if (int rc = gz_prepare(c)) return rc; }
@@ -1089,6 +1172,36 @@ int yield_reads(scs_ctx* c, SlabConsumer& sink) {
         for (int b = 0; b < 2; b++) SCS_CUDA(c, c->gz.slab[b][f].reserve(slab + 64));
     }
 
+    // packed slabs expanded by host threads (wire.h, scs_params.host_expand): the device slabs also hold the split table and the
+    // 3-byte prefix of every record, the packed slabs land in a ring of pinned wire slots and the pool expands them into the
+    // consumer's slots
+    const int hx = c->P.host_expand;
+    const bool hybrid = !gz && relay < 0 && R.nslots > 0 && sink.takes_expanded() && (hx == 1 || hx == 2 || (hx < 0 && c->P.world == 1));
+    const int Rw = 3;
+    const uint64_t split_max = (batch / wire::kSplitEvery + 2) * sizeof(wire::Split), wcap = slab + 3 * batch + split_max + 64;
+    if (hybrid) {
+        for (int b = 0; b < 2; b++) for (int f = 0; f < nfiles; f++) SCS_CUDA(c, c->slab_dev[b][f].reserve(wcap));
+        if (c->wire_cap < wcap) {
+            for (int f = 0; f < 2; f++) { for (char* q : c->wire_host[f]) cudaFreeHost(q); c->wire_host[f].clear(); }
+            c->wire_cap = wcap;
+        }
+        for (int f = 0; f < nfiles; f++) while ((int)c->wire_host[f].size() < Rw) {
+            char* q = nullptr;
+            SCS_CUDA(c, cudaMallocHost((void**)&q, c->wire_cap));
+            c->wire_host[f].push_back(q);
+        }
+        if (!c->pool) {
+            int n = c->P.expand_threads;
+            if (n <= 0) {
+                cpu_set_t set; CPU_ZERO(&set);
+                n = sched_getaffinity(0, sizeof(set), &set) == 0 ? CPU_COUNT(&set) - 1 : 1;
+            }
+            c->pool = new ExpandPool(c->P.device, std::max(1, n));
+        }
+    }
+    // per consumer slot: the expansion job that writes its text (declared before the guard, which drains the pool first)
+    std::vector<ExpandJob> jobs(Rn);
+
     StageGuard G(c);   // from here on every return drains the streams and frees the events
     if (R.nslots == 0) {   // gzip of an empty output: the 28-byte end-of-file member, so that the file is a valid (empty) gzip stream
         static const uint8_t eof[28] = {31, 139, 8, 4, 0, 0, 0, 0, 0, 255, 6, 0, 66, 67, 2, 0, 27, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
@@ -1112,6 +1225,8 @@ int yield_reads(scs_ctx* c, SlabConsumer& sink) {
     for (int b = 0; b < 2; b++) ecopy[b] = G.make(cudaEventDisableTiming);
     std::vector<cudaEvent_t> eslot(Rn); for (int i = 0; i < Rn; i++) eslot[i] = G.make(cudaEventDisableTiming);
     if (relay >= 0) cudaSetDevice(dev_self);
+    cudaEvent_t tc[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};   // around the copies of buffer b: the link rate
+    if (hybrid) for (int b = 0; b < 2; b++) { tc[b][0] = G.make(cudaEventDefault); tc[b][1] = G.make(cudaEventDefault); }
     cudaStream_t st_d2h = relay >= 0 ? c->st_relay : c->st_copy;
     double msk = 0, mse = 0;
     auto harvest = [&](int b) {   // kernel times of the slab that used buffer b (its events are complete: a later event was waited for)
@@ -1124,7 +1239,37 @@ int yield_reads(scs_ctx* c, SlabConsumer& sink) {
     // ---- per slab: emit (staging + sizes) -> scans -> compaction into the packed device slab -> D2H into a pinned ring slot.
     // Software-pipelined on the host: slab k is launched before the host waits for the byte totals of slab k-1, so the kernels
     // run back to back; the consumer is serviced in between.
-    struct DevSlab { bool launched = false; uint64_t k = 0; } dv[2];
+    struct DevSlab { bool launched = false, packed = false; uint64_t k = 0, m = 0; } dv[2];
+    // per-slab choice (host_expand = -1): the path, text over the link or packed + host expansion, whose queue drains sooner with
+    // this slab added: (bytes queued on the copy stream + the slab's text) / link rate against (text queued on the pool + the
+    // slab's text) / expansion rate. Link rate from the copy events, expansion rate from the pool. The emit kernel keeps both
+    // sides busy, so this greedy rule settles where the link and the host threads finish together.
+    double link_rate = 50e9, wire_ratio = 0.53, last_text = (double)batch * (nfiles == 2 ? 2.0 : 1.0) * (double)(2 * T.RL + 30);
+    uint64_t copy_pend[2] = {0, 0}, wire_k = 0;
+    ExpandJob* wjob[3] = {nullptr, nullptr, nullptr}; uint64_t wseq[3] = {0, 0, 0};
+    auto harvest_link = [&]() {
+        for (int b = 0; b < 2; b++) {
+            if (!copy_pend[b]) continue;
+            cudaError_t q = cudaEventQuery(tc[b][1]);
+            if (q == cudaErrorNotReady) { (void)cudaGetLastError(); continue; }
+            float ms = 0;
+            if (q == cudaSuccess && cudaEventElapsedTime(&ms, tc[b][0], tc[b][1]) == cudaSuccess && ms > 0.05f)
+                link_rate = 0.75 * link_rate + 0.25 * (double)copy_pend[b] / (ms * 1e-3);
+            copy_pend[b] = 0;
+        }
+    };
+    auto choose_packed = [&](uint64_t kk, int b) -> bool {
+        if (!hybrid) return false;
+        if (hx == 1) return true;
+        if (hx == 2) return (kk & 1) != 0;
+        harvest_link();
+        const int o = b ^ 1;   // the slab launched before this one: its path is chosen, its bytes are not queued yet
+        const double T = last_text;
+        double qlink = (double)(copy_pend[0] + copy_pend[1]), qpool = (double)c->pool->queued_text();
+        if (dv[o].launched) { if (dv[o].packed) { qpool += T; qlink += wire_ratio * T; } else qlink += T; }
+        const double P = c->pool->rate() > 0 ? c->pool->rate() : 2e9 * c->pool->threads();
+        return (qpool + T) / P < (qlink + T) / link_rate;
+    };
     auto finalize = [&](int b) -> int {   // the kernels of device buffer b were launched: wait for the byte totals, queue the copy behind the compaction
         if (!dv[b].launched) return SCS_OK;
         SCS_CUDA(c, cudaEventSynchronize(etotb[b]));
@@ -1137,6 +1282,41 @@ int yield_reads(scs_ctx* c, SlabConsumer& sink) {
         SCS_CUDA(c, cudaStreamWaitEvent(c->st_copy, ekern[b], 0));
         char* p[2] = {nullptr, nullptr};
         for (int f = 0; f < nfiles; f++) p[f] = c->ring_host[f][slot] + (sink.phase(f) & 4095);
+        c->stats.slabs++;
+        last_text = (double)(tot[0] + tot[1]);
+        if (dv[b].packed) {
+            // packed slab: split table + records into the next pinned wire slot, then the pool expands it into the consumer's slot
+            const uint32_t nsplit = (uint32_t)((dv[b].m + wire::kSplitEvery - 1) / wire::kSplitEvery);
+            const uint64_t wtot[2] = {W.htotals[8 + 2 * b], nfiles == 2 ? W.htotals[8 + 2 * b + 1] : 0};
+            uint64_t cb[2] = {0, 0};
+            for (int f = 0; f < nfiles; f++) {
+                cb[f] = tot[f] ? nsplit * sizeof(wire::Split) + wtot[f] : 0;
+                if (cb[f] > wcap) return c->fail(SCS_E_NOMEM, "packed FASTQ slab too small for one batch (raise slab_bytes)");
+            }
+            const int ws = (int)(wire_k++ % Rw);
+            if (wjob[ws] && wjob[ws]->seq == wseq[ws] && c->pool->wait(wjob[ws])) return c->fail(SCS_E_STATE, "host expansion of a packed FASTQ slab failed");
+            SCS_CUDA(c, cudaEventRecord(tc[b][0], c->st_copy));
+            for (int f = 0; f < nfiles; f++)
+                if (cb[f]) SCS_CUDA(c, cudaMemcpyAsync(c->wire_host[f][ws], c->slab_dev[b][f].p, cb[f], cudaMemcpyDeviceToHost, c->st_copy));
+            SCS_CUDA(c, cudaEventRecord(tc[b][1], c->st_copy)); copy_pend[b] = cb[0] + cb[1];
+            SCS_CUDA(c, cudaEventRecord(ecopy[b], c->st_copy)); SCS_CUDA(c, cudaEventRecord(eslot[slot], c->st_copy));
+            if (tot[0] + tot[1]) wire_ratio = 0.75 * wire_ratio + 0.25 * (double)(cb[0] + cb[1]) / (double)(tot[0] + tot[1]);
+            ExpandJob& J = jobs[slot];
+            J.landed = eslot[slot]; J.qchar0 = 33 + (int)c->wire_qlo;
+            for (int f = 0; f < 2; f++) {
+                const bool on = f < nfiles && tot[f];
+                J.wire[f] = on ? reinterpret_cast<const uint8_t*>(c->wire_host[f][ws]) : nullptr; J.nsplit[f] = on ? nsplit : 0;
+                J.wire_bytes[f] = on ? wtot[f] : 0; J.text_bytes[f] = on ? tot[f] : 0; J.out[f] = p[f];
+            }
+            c->pool->submit(&J);
+            wjob[ws] = &J; wseq[ws] = J.seq;
+            c->stats.fastq_bytes[0] += tot[0]; c->stats.fastq_bytes[1] += tot[1];
+            c->stats.plain_bytes[0] += tot[0]; c->stats.plain_bytes[1] += tot[1];
+            c->stats.link_bytes[0] += cb[0]; c->stats.link_bytes[1] += cb[1]; c->stats.slabs_packed++;
+            if (sink.submit_expanded(slot, c->pool, &J, p, tot)) return c->fail(SCS_E_IO, "FASTQ sink failed");
+            return SCS_OK;
+        }
+        if (hybrid) SCS_CUDA(c, cudaEventRecord(tc[b][0], c->st_copy));
         if (relay < 0) {
             for (int f = 0; f < nfiles; f++)
                 if (tot[f]) SCS_CUDA(c, cudaMemcpyAsync(p[f], gz ? c->gz.slab[b][f].p : c->slab_dev[b][f].p, tot[f], cudaMemcpyDeviceToHost, c->st_copy));
@@ -1152,8 +1332,10 @@ int yield_reads(scs_ctx* c, SlabConsumer& sink) {
         }
         cudaError_t er = cudaEventRecord(ecopy[b], st_d2h);
         if (er == cudaSuccess) er = cudaEventRecord(eslot[slot], st_d2h);
+        if (er == cudaSuccess && hybrid) { er = cudaEventRecord(tc[b][1], st_d2h); copy_pend[b] = tot[0] + tot[1]; }
         if (relay >= 0) cudaSetDevice(dev_self);
         SCS_CUDA(c, er);
+        c->stats.link_bytes[0] += tot[0]; c->stats.link_bytes[1] += tot[1];
         c->stats.fastq_bytes[0] += tot[0]; c->stats.fastq_bytes[1] += tot[1];
         c->stats.plain_bytes[0] += plain[0]; c->stats.plain_bytes[1] += plain[1];
         if (sink.submit(slot, eslot[slot], p, tot)) return c->fail(SCS_E_IO, "FASTQ sink failed");
@@ -1165,6 +1347,7 @@ int yield_reads(scs_ctx* c, SlabConsumer& sink) {
         const uint64_t m = std::min(batch, slot_hi - s0);
         A.slot0 = s0; A.nslots = m;
         harvest(b);
+        const bool packed = choose_packed(k, b);
         SCS_CUDA(c, cudaEventRecord(tq[b][0], c->st));
         SCS_CUDA(c, cudaMemsetAsync(W.size1.p, 0, (m + 1) * 4, c->st));
         if (nfiles == 2) SCS_CUDA(c, cudaMemsetAsync(W.size2.p, 0, (m + 1) * 4, c->st));
@@ -1179,7 +1362,20 @@ int yield_reads(scs_ctx* c, SlabConsumer& sink) {
         if (nfiles == 2) { if (int rc = scan_u32_noalloc(c, W.size2.p, W.off2.p, m, W.scan.p + 2048 + 8, plain_tot + 1)) return rc; }
         SCS_CUDA(c, cudaEventRecord(tq[b][3], c->st));   // kernel time of the slab without the compaction (~0.05 ms), which may wait for a copy
         const unsigned cgrid = (unsigned)std::min<uint64_t>((m + 7) / 8, (uint64_t)sms * 16);
-        if (!gz) {
+        if (packed) {
+            // wire bytes per record and their scan (total into the mapped slot 8 + 2b + f), then the packed slab behind its split table
+            for (int f = 0; f < nfiles; f++) {
+                wire_size_kernel<<<cgrid, 256, 0, c->st>>>(W.stage[f].p, stride, f ? W.size2.p : W.size1.p, m, c->wire_qlo, W.wsize[f].p); SCS_LAUNCHED(c);
+                if (int rc = scan_u32_noalloc(c, W.wsize[f].p, W.woff[f].p, m, W.scan.p + (f ? 2048 + 8 : 0), W.dtotals_mapped + 8 + 2 * b + f)) return rc;
+            }
+            SCS_CUDA(c, cudaEventRecord(etotb[b], c->st));
+            SCS_CUDA(c, cudaStreamWaitEvent(c->st, ecopy[b], 0));   // device slab b is free once the copy of the slab two back is done
+            for (int f = 0; f < nfiles; f++) {
+                pack_records_kernel<<<cgrid, 256, 0, c->st>>>(W.stage[f].p, stride, f ? W.size2.p : W.size1.p, f ? W.off2.p : W.off1.p, W.woff[f].p, m, c->wire_qlo,
+                                                              c->slab_dev[b][f].p, wcap, W.flags.p);
+                SCS_LAUNCHED(c);
+            }
+        } else if (!gz) {
             SCS_CUDA(c, cudaEventRecord(etotb[b], c->st));
             // the packed device slab b is free once the copy of the slab two back is done
             SCS_CUDA(c, cudaStreamWaitEvent(c->st, ecopy[b], 0));
@@ -1205,7 +1401,7 @@ int yield_reads(scs_ctx* c, SlabConsumer& sink) {
         }
         timed[b] = true;
         SCS_CUDA(c, cudaEventRecord(ekern[b], c->st));
-        dv[b].launched = true; dv[b].k = k;
+        dv[b].launched = true; dv[b].k = k; dv[b].packed = packed; dv[b].m = m;
         if (int rc = finalize(b ^ 1)) return rc;   // slab k-1: totals known -> copy queued behind its compaction
         if (sink.service()) return c->fail(SCS_E_IO, "FASTQ sink failed");
     }
